@@ -20,6 +20,12 @@ roofline / cpu_baseline / clocks: see DESIGN.md "Measurement".
 cannot be compiled in this image, so this arm times the oracle port
 (oracle/sais_oracle.c: restated sais() + lcp_lens()) on one host core (the
 reference is single-threaded), each step on a bounded prefix of the workload.
+
+--dump-outputs DIR: after the timed steps, writes the SA and LCP arrays of the last
+device-resident step (rank 0) as DIR/sa.npy and DIR/lcp.npy (float64, exact for
+u32 values).  Above DUMP_ENTRIES entries both arrays are sampled at the same
+seeded set of indices.  The input text is seeded too, so two builds of the project
+run with the same arguments can be compared entry for entry.
 """
 import argparse
 import json
@@ -34,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no bytecode caches written into it
 
 from suffix_b200 import gen  # noqa: E402
 
@@ -41,6 +48,8 @@ N_TEXT = 100_000_000
 METRIC = "MB/s input text indexed (SA+LCP build)"
 UNIT = "MB/s"
 WORKLOAD = "100 MB synthetic DNA (sigma=4) SA-IS build + LCP, G_dna seed 0x5AFE5EED0000D7A4"
+DUMP_ENTRIES = 3_000_000                # per dumped array: 2 x 3e6 float64 = 48 MB, under a 64 MB budget
+DUMP_SEED = 0x5AFE5EED0000D0D0
 
 
 def _peaks():
@@ -195,6 +204,18 @@ def run_reference(args):
     }
     _emit(json.dumps(out))
     return 0
+
+
+def _dump_outputs(out_dir, arrays):
+    """Writes each named u32 array as out_dir/<name>.npy in float64.  Arrays longer than
+    DUMP_ENTRIES are all sampled at the same sorted, seeded indices (fixed for a given n)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    idx = None
+    if n > DUMP_ENTRIES:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ENTRIES, replace=False))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), (a if idx is None else a[idx]).astype(np.float64))
 
 
 def _config(n, world):
@@ -454,6 +475,9 @@ def run_gpu(args):
             cpu["gpu_matches_oracle_e2e"] = bool(np.array_equal(h_sa.numpy().view(np.uint32), sa_cpu) and
                                                  np.array_equal(h_lcp.numpy().view(np.uint32), lcp_cpu))
             cpu["compared"] = "SA and LCP, all %d entries each, device-resident result and host-API result" % n
+        if args.dump_outputs:           # d_sa / d_lcp still hold the last device-resident step's result
+            _dump_outputs(args.dump_outputs, {"sa": d_sa.cpu().numpy().view(np.uint32),
+                                              "lcp": d_lcp.cpu().numpy().view(np.uint32)})
         out = {
             "metric": METRIC, "value": round(value, 2), "unit": UNIT, "n_gpus": world, "steps": steps,
             "warmup": warm, "ms_per_step": round(ms_dev / steps, 3), "higher_is_better": True,
@@ -505,7 +529,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-sharded", action="store_true", help="N > 1: skip the sharded config-5 record")
     ap.add_argument("--shard-bytes", type=int, default=1_000_000_000, help="N > 1: bytes per GPU of the sharded text")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's SA and LCP (rank 0; sampled, see DUMP_ENTRIES) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
