@@ -138,6 +138,44 @@ int b200sa_doc_ids_dev(b200sa_ctx *ctx, const uint32_t *d_pos, uint64_t count,
 int b200sa_lcp_intervals_dev(b200sa_ctx *ctx, const uint32_t *d_lcp, uint64_t n,
                              uint32_t *d_psv, uint32_t *d_nsv, void *stream);
 
+/* ---- suffix tree (SURVEY.md 8f-5; reference suffix_tree/src/lib.rs) ----
+ * The tree the reference's SuffixTree::new / from_suffix_table builds, as structure-of-arrays
+ * indexed by preorder id (children in first-byte order = the reference's preorder()):
+ *   parent     parent id; 0xFFFFFFFF for the root (id 0)
+ *   depth      string depth (length of the path label from the root)
+ *   lo, hi     the node's suffixes below it are table[lo, hi) (the root: [0, n))
+ *   end        one past the last id of its subtree; children of u are u+1, then end[c]
+ *              repeatedly while < end[u]
+ *   nchildren  number of children
+ * The node's label is text[sa[lo] + depth[parent], sa[lo] + depth).  Like the reference there
+ * is no sentinel: a node has a terminal iff depth == n - sa[lo] (suffix sa[lo]), or it is the
+ * root (suffix n, empty label); such a leaf may still have children, when its suffix is a
+ * prefix of the next one.  There are at most max(2n, 1) nodes.
+ * Node ids are u32, so n <= B200SA_TREE_MAX_N; above it both entry points return
+ * B200SA_ERR_TOO_LARGE before touching any pointer. */
+#define B200SA_TREE_MAX_N 0x7FFFFFFFull
+typedef struct {
+    uint32_t *parent, *depth, *lo, *hi, *end, *nchildren;
+} b200sa_tree;
+
+/* Device-resident construction: d_sa and d_lcp (n u32 each, LCP as lcp_lens) are trusted like
+ * SuffixTable::from_parts: they must be the table and LCP array of the n bytes at d_text (the
+ * tree is built from them alone; d_text names the text they index).  The six arrays of d_out
+ * are device buffers of max(2n, 1) entries; *num_nodes gets the exact node count (one small
+ * device-to-host read).  n = 0 and n = 1 launch no kernels. */
+int b200sa_suffix_tree_dev(b200sa_ctx *ctx, const uint8_t *d_text, uint64_t n, const uint32_t *d_sa,
+                           const uint32_t *d_lcp, const b200sa_tree *d_out, uint64_t *num_nodes, void *stream);
+
+/* Host twin; the six arrays of h_out are host buffers of max(2n, 1) entries.
+ *   sa_given == 0: SuffixTree::new -- SA and LCP are built on the device and the SA is written
+ *                  to sa[0..n) (labels and terminals need it);
+ *   sa_given != 0: SuffixTree::from_suffix_table -- sa[0..n) is read and checked to be a
+ *                  permutation of 0..n-1 (B200SA_ERR_BAD_ARG otherwise), the LCP is computed
+ *                  as b200sa_lcp does.
+ * The LCP array stays on the device. */
+int b200sa_suffix_tree(b200sa_ctx *ctx, const uint8_t *text, uint64_t n, uint32_t *sa, int sa_given,
+                       const b200sa_tree *h_out, uint64_t *num_nodes);
+
 /* ---- multi-GPU: communicator + sharded LMS-suffix sort (SURVEY.md 8e, config 5) ----
  * One process (or thread) and one context per GPU.  NCCL is resolved at run time
  * (the copy already loaded in the process, else libnccl.so.2); the single-GPU entry

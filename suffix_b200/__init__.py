@@ -5,3 +5,4 @@ there is no CPU fallback."""
 from ._lib import B200SAError, Context, default_context  # noqa: F401
 from .table import SuffixTable  # noqa: F401
 from .generalized import GeneralizedSuffixTable  # noqa: F401,E402
+from .tree import Node, SuffixTree  # noqa: F401,E402

@@ -30,6 +30,15 @@ class ShardStats(ctypes.Structure):
                 ("kc", ctypes.c_uint32), ("nranks", ctypes.c_uint32), ("rank", ctypes.c_uint32), ("reserved", ctypes.c_uint32)]
 
 
+class Tree(ctypes.Structure):
+    """b200sa_tree: the six node arrays (host or device pointers)."""
+    _fields_ = [(f, ctypes.c_void_p) for f in ("parent", "depth", "lo", "hi", "end", "nchildren")]
+
+
+TREE_FIELDS = tuple(f for f, _ in Tree._fields_)
+TREE_MAX_N = 0x7FFFFFFF   # B200SA_TREE_MAX_N
+
+
 _lib = None
 
 
@@ -63,6 +72,8 @@ def lib():
         "b200sa_doc_ids_dev": ([vp, vp, u64, vp, u32, vp, vp, vp], ci),
         "b200sa_lcp_intervals_dev": ([vp, vp, u64, vp, vp, vp], ci),
         "b200sa_lcp_sharded": ([vp, vp, u64, vp, vp, ci, vp], ci),
+        "b200sa_suffix_tree_dev": ([vp, vp, u64, vp, vp, ctypes.POINTER(Tree), ctypes.POINTER(u64), vp], ci),
+        "b200sa_suffix_tree": ([vp, vp, u64, vp, ci, ctypes.POINTER(Tree), ctypes.POINTER(u64)], ci),
         "b200sa_last_stats": ([vp, ctypes.POINTER(Stats)], ci),
         "b200sa_set_timing": ([vp, ci], ci),
         "b200sa_last_phase_times": ([vp, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_float), ci], ci),
@@ -192,6 +203,31 @@ class Context:
 
     def lcp_sharded(self, d_text: int, n: int, d_sa: int, d_lcp: int, replicated: bool = False, stream: int = 0):
         self._check(lib().b200sa_lcp_sharded(self._h, d_text, n, d_sa, d_lcp, 1 if replicated else 0, stream))
+
+    def suffix_tree_dev(self, d_text: int, n: int, d_sa: int, d_lcp: int, d_out: dict, stream: int = 0) -> int:
+        """b200sa_suffix_tree_dev: d_out maps each of TREE_FIELDS to a device pointer of
+        max(2n, 1) u32; returns the node count."""
+        k = ctypes.c_uint64(0)
+        tree = Tree(*(d_out[f] for f in TREE_FIELDS))
+        self._check(lib().b200sa_suffix_tree_dev(self._h, d_text, n, d_sa, d_lcp, ctypes.byref(tree),
+                                                 ctypes.byref(k), stream))
+        return int(k.value)
+
+    def suffix_tree(self, text: np.ndarray, sa: np.ndarray = None):
+        """b200sa_suffix_tree -> (sa, {field: u32 array of the node count}).  sa=None builds the
+        table on the device (SuffixTree::new); a given table is checked (from_suffix_table)."""
+        n = len(text)
+        cap = max(2 * n, 1)
+        out = {f: np.empty(cap, dtype=np.uint32) for f in TREE_FIELDS}
+        given = sa is not None
+        sa = np.ascontiguousarray(sa, dtype=np.uint32) if given else np.empty(n, dtype=np.uint32)
+        if len(sa) != n:
+            raise ValueError("table length %d != text length %d" % (len(sa), n))
+        k = ctypes.c_uint64(0)
+        tree = Tree(*(out[f].ctypes.data for f in TREE_FIELDS))
+        self._check(lib().b200sa_suffix_tree(self._h, text.ctypes.data, n, sa.ctypes.data, 1 if given else 0,
+                                             ctypes.byref(tree), ctypes.byref(k)))
+        return sa, {f: a[:k.value] for f, a in out.items()}
 
     # ---- introspection
     def set_timing(self, on: bool):

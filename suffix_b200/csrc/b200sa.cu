@@ -28,6 +28,7 @@
 #include "pipeline_kernels.cuh"
 #include "lms_sort.cuh"
 #include "shard.cuh"
+#include "tree.cuh"
 #include "nccl_dyn.h"
 
 using namespace b200sa;
@@ -78,6 +79,7 @@ struct b200sa_ctx {
     bool comm_owned = false;
     int nranks = 1, comm_rank = 0;
     DevBuf sh_a, sh_b, sh_c, sh_d, sh_e, sh_f, sh_small;
+    DevBuf tree;                      // staging of the host suffix-tree API (six node arrays)
     bool lms_asc_ready = false;       // c->lmspos / c->lmsrank (text order) valid for the current text
     uint32_t scan_epoch = 0, scan_tiles_cap = 0;
     bool l2_persist = false;          // access policy window for the packed text (B200SA_L2PERSIST)
@@ -1225,7 +1227,7 @@ void b200sa_ctx_destroy(b200sa_ctx *c) {
     DevBuf *bufs[] = {&c->text, &c->sa, &c->lcp, &c->pred, &c->stype, &c->lmsb, &c->lmsrank, &c->lmspos, &c->lmslist,
                       &c->lmspred, &c->sorted, &c->flag, &c->reduced, &c->sa_r, &c->blkstate, &c->carry, &c->tables,
                       &c->small, &c->scan_partial, &c->radix_cnt, &c->blkcnt, &c->k32b, &c->k64a, &c->k64b, &c->v0,
-                      &c->v1, &c->p0, &c->p1, &c->g0, &c->g1, &c->rank, &c->isa, &c->qbuf, &c->os_hist, &c->os_status, &c->packed, &c->phik, &c->phiv, &c->runscr, &c->plcp_samp, &c->scan_state, &c->cls_state, &c->lmsdesc, &c->steplog, &c->hist_copies, &c->sh_a, &c->sh_b, &c->sh_c, &c->sh_d, &c->sh_e, &c->sh_f, &c->sh_small};
+                      &c->v1, &c->p0, &c->p1, &c->g0, &c->g1, &c->rank, &c->isa, &c->qbuf, &c->os_hist, &c->os_status, &c->packed, &c->phik, &c->phiv, &c->runscr, &c->plcp_samp, &c->scan_state, &c->cls_state, &c->lmsdesc, &c->steplog, &c->hist_copies, &c->sh_a, &c->sh_b, &c->sh_c, &c->sh_d, &c->sh_e, &c->sh_f, &c->sh_small, &c->tree};
     for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
     for (cudaEvent_t e : c->event_pool) cudaEventDestroy(e);
     if (c->h_pin) cudaFreeHost(c->h_pin);
@@ -1456,6 +1458,25 @@ int b200sa_doc_ids_dev(b200sa_ctx *c, const uint32_t *d_pos, uint64_t count, con
     return end_call(c);
 }
 
+// Minima of d_lcp over blocks of 32^k entries (in c->qbuf), shared by every k_ansv launch on d_lcp.
+static int ansv_levels(b200sa_ctx *c, const uint32_t *d_lcp, uint64_t n, AnsvLevels *L) {
+    memset(L, 0, sizeof *L);
+    L->lv[0] = d_lcp; L->cnt[0] = n; L->nlev = 1;
+    uint64_t total = 0;
+    for (uint64_t k = (n + 31) / 32; ; k = (k + 31) / 32) { total += k; if (k <= 32) break; }
+    TRY(ensure(c, c->qbuf, (total + 64) * 4));
+    uint32_t *lvbuf = ptr<uint32_t>(c->qbuf);
+    uint64_t cnt = n;
+    while (cnt > 32 && L->nlev < 8) {
+        uint64_t nxt = (cnt + 31) / 32;
+        LAUNCH(c, k_min32, cdiv(nxt, BLK), L->lv[L->nlev - 1], cnt, lvbuf);
+        L->lv[L->nlev] = lvbuf; L->cnt[L->nlev] = nxt; L->nlev++;
+        lvbuf += nxt;
+        cnt = nxt;
+    }
+    return B200SA_OK;
+}
+
 int b200sa_lcp_intervals_dev(b200sa_ctx *c, const uint32_t *d_lcp, uint64_t n, uint32_t *d_psv, uint32_t *d_nsv,
                              void *stream) {
     if (!c || (n > 0 && (!d_lcp || !d_psv || !d_nsv))) return B200SA_ERR_BAD_ARG;
@@ -1464,23 +1485,143 @@ int b200sa_lcp_intervals_dev(b200sa_ctx *c, const uint32_t *d_lcp, uint64_t n, u
     begin_call(c, stream);
     if (n == 0) return end_call(c);
     AnsvLevels L;
-    memset(&L, 0, sizeof L);
-    L.lv[0] = d_lcp; L.cnt[0] = n; L.nlev = 1;
-    uint64_t total = 0;
-    for (uint64_t k = (n + 31) / 32; ; k = (k + 31) / 32) { total += k; if (k <= 32) break; }
-    TRY(ensure(c, c->qbuf, (total + 64) * 4));
-    uint32_t *lvbuf = ptr<uint32_t>(c->qbuf);
-    uint64_t cnt = n;
-    while (cnt > 32 && L.nlev < 8) {
-        uint64_t nxt = (cnt + 31) / 32;
-        LAUNCH(c, k_min32, cdiv(nxt, BLK), L.lv[L.nlev - 1], cnt, lvbuf);
-        L.lv[L.nlev] = lvbuf; L.cnt[L.nlev] = nxt; L.nlev++;
-        lvbuf += nxt;
-        cnt = nxt;
-    }
-    LAUNCH(c, k_ansv, cdiv(n, BLK), L, n, d_psv, d_nsv);
+    TRY(ansv_levels(c, d_lcp, n, &L));
+    LAUNCH(c, k_ansv<true>, cdiv(n, BLK), L, n, d_psv, d_nsv);
     CU_TRY(c, cudaGetLastError());
     return end_call(c);
+}
+
+// ------------------------------------------------------------ suffix tree (SURVEY 8f-5, tree.cuh)
+// Node arrays of the tree of an n-byte text from its SA and LCP on the device; *count = nodes.
+// Scratch: p0 psv, p1 nsv, g0 pse, g1 head -> node id, rank e / base, v0 v1 k32b isa the sort.
+static int tree_dev(b200sa_ctx *c, uint64_t n, const uint32_t *d_sa, const uint32_t *d_lcp, const b200sa_tree *o,
+                    uint64_t *count) {
+    if (n <= 1) {
+        // root (and the leaf of suffix 0): no launches, six tiny copies through the pinned words
+        static const uint32_t one[6][2] = {{TREE_NONE, 0}, {0, 1}, {0, 0}, {1, 1}, {2, 2}, {1, 0}};
+        uint32_t *const dst[6] = {o->parent, o->depth, o->lo, o->hi, o->end, o->nchildren};
+        for (int f = 0; f < 6; f++) {
+            c->h_pin[2 * f] = one[f][0];
+            c->h_pin[2 * f + 1] = one[f][1];
+        }
+        if (n == 0) { c->h_pin[6] = 0; c->h_pin[8] = 1; c->h_pin[10] = 0; }      // hi, end, nchildren of a lone root
+        for (int f = 0; f < 6; f++)
+            CU_TRY(c, cudaMemcpyAsync(dst[f], c->h_pin + 2 * f, (n + 1) * 4, cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        *count = n + 1;
+        return B200SA_OK;
+    }
+    uint32_t n32 = (uint32_t)n;
+    TRY(ensure(c, c->p0, n * 4));
+    TRY(ensure(c, c->p1, n * 4));
+    TRY(ensure(c, c->g0, n * 4));
+    TRY(ensure(c, c->g1, n * 4));
+    TRY(ensure(c, c->rank, (n + 1) * 4));
+    TRY(ensure(c, c->v0, n * 4));
+    TRY(ensure(c, c->v1, n * 4));
+    TRY(ensure(c, c->k32b, n * 4));
+    TRY(ensure(c, c->isa, n * 4));
+    TRY(ensure(c, c->small, 4096));
+    uint32_t *psv = ptr<uint32_t>(c->p0), *nsv = ptr<uint32_t>(c->p1), *pse = ptr<uint32_t>(c->g0);
+    uint32_t *headid = ptr<uint32_t>(c->g1), *base = ptr<uint32_t>(c->rank), *d_m = ptr<uint32_t>(c->small) + 40;
+    TRY(mark(c, "tree_ansv"));
+    AnsvLevels L;
+    TRY(ansv_levels(c, d_lcp, n, &L));
+    LAUNCH(c, k_ansv<true>, cdiv(n, BLK), L, n, psv, nsv);
+    LAUNCH(c, k_ansv<false>, cdiv(n, BLK), L, n, pse, (uint32_t *)nullptr);
+    TRY(mark(c, "tree_heads"));
+    TreeIn t{d_sa, d_lcp, psv, nsv, pse, n32};
+    TRY((dev_scan<OpSum>(c, InTreeHead{d_sa, d_lcp, psv, pse, n32}, OutTreeHead{psv, ptr<uint32_t>(c->v0), ptr<uint32_t>(c->v1), n32},
+                         n, d_m)));
+    TRY(read_words(c, d_m, 1));
+    uint32_t m = c->h_pin[0];
+    TRY(mark(c, "tree_sort"));
+    uint32_t *key = ptr<uint32_t>(c->v0), *val = ptr<uint32_t>(c->v1);
+    TRY(sort_pairs<uint32_t>(c, key, val, ptr<uint32_t>(c->k32b), ptr<uint32_t>(c->isa), m, bit_length(n - 1),
+                             &key, &val));
+    TRY(mark(c, "tree_base"));
+    CU_TRY(c, cudaMemsetAsync(base, 0, (n + 1) * 4, c->stream));
+    if (m) LAUNCH(c, k_tree_bucket_end, cdiv(m, BLK), key, m, base);
+    TRY((dev_scan<OpMax>(c, InArray{base}, OutTreeBase{base}, n + 1, nullptr)));
+    TRY(mark(c, "tree_nodes"));
+    uint64_t nodes = 1 + n + (uint64_t)m;
+    TreeOut to{o->parent, o->depth, o->lo, o->hi, o->end, o->nchildren};
+    CU_TRY(c, cudaMemsetAsync(o->nchildren, 0, nodes * 4, c->stream));
+    if (m) LAUNCH(c, k_tree_internal, cdiv(m, BLK), t, key, val, m, base, headid, to);
+    LAUNCH(c, k_tree_link, cdiv(n, BLK), t, base, headid, to);
+    TRY(mark(c, "end"));
+    CU_TRY(c, cudaGetLastError());
+    *count = nodes;
+    return B200SA_OK;
+}
+
+int b200sa_suffix_tree_dev(b200sa_ctx *c, const uint8_t *d_text, uint64_t n, const uint32_t *d_sa,
+                           const uint32_t *d_lcp, const b200sa_tree *d_out, uint64_t *num_nodes, void *stream) {
+    if (!c) return B200SA_ERR_BAD_ARG;
+    if (n > B200SA_TREE_MAX_N) { c->last_error = "text longer than B200SA_TREE_MAX_N = 2^31-1 bytes"; return B200SA_ERR_TOO_LARGE; }
+    if (!d_out || !num_nodes || (n > 0 && (!d_text || !d_sa || !d_lcp)) || !d_out->parent || !d_out->depth ||
+        !d_out->lo || !d_out->hi || !d_out->end || !d_out->nchildren)
+        return B200SA_ERR_BAD_ARG;
+    CU_TRY(c, cudaSetDevice(c->device));
+    begin_call(c, stream);
+    TRY(tree_dev(c, n, d_sa, d_lcp, d_out, num_nodes));
+    return end_call(c);
+}
+
+static int host_tree_inner(b200sa_ctx *c, const uint8_t *text, uint64_t n, uint32_t *sa, int sa_given,
+                           const b200sa_tree *h, uint64_t *num_nodes) {
+    CU_TRY(c, cudaSetDevice(c->device));
+    begin_call(c, nullptr);
+    memset(&c->stats, 0, sizeof c->stats);
+    c->stats.n = n;
+    size_t cap = n ? 2 * n : 1;
+    TRY(ensure(c, c->tree, 6 * cap * 4));
+    uint32_t *tb = ptr<uint32_t>(c->tree);
+    b200sa_tree d{tb, tb + cap, tb + 2 * cap, tb + 3 * cap, tb + 4 * cap, tb + 5 * cap};
+    const uint32_t *d_sa = nullptr, *d_lcp = nullptr;
+    if (n >= 1) {
+        TRY(ensure(c, c->text, n));
+        TRY(ensure(c, c->sa, n * 4));
+        TRY(ensure(c, c->lcp, n * 4));
+        TRY(mark(c, "h2d"));
+        CU_TRY(c, cudaMemcpyAsync(c->text.p, text, n, cudaMemcpyHostToDevice, c->stream));
+        if (sa_given) {
+            // SuffixTree::from_suffix_table: the table comes from the caller, lcp_dev checks it
+            CU_TRY(c, cudaMemcpyAsync(c->sa.p, sa, n * 4, cudaMemcpyHostToDevice, c->stream));
+            TRY(lcp_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa), ptr<uint32_t>(c->lcp), false));
+        } else {
+            TRY(build_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa)));
+            TRY(lcp_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa), ptr<uint32_t>(c->lcp), n >= 2));
+        }
+        d_sa = ptr<uint32_t>(c->sa);
+        d_lcp = ptr<uint32_t>(c->lcp);
+    }
+    uint64_t k = 0;
+    TRY(tree_dev(c, n, d_sa, d_lcp, &d, &k));
+    TRY(mark(c, "d2h_tree"));
+    if (!sa_given && n) CU_TRY(c, cudaMemcpyAsync(sa, c->sa.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
+    uint32_t *const src[6] = {d.parent, d.depth, d.lo, d.hi, d.end, d.nchildren};
+    uint32_t *const dst[6] = {h->parent, h->depth, h->lo, h->hi, h->end, h->nchildren};
+    for (int f = 0; f < 6; f++) CU_TRY(c, cudaMemcpyAsync(dst[f], src[f], k * 4, cudaMemcpyDeviceToHost, c->stream));
+    TRY(mark(c, "end"));
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    *num_nodes = k;
+    return end_call(c);
+}
+
+int b200sa_suffix_tree(b200sa_ctx *c, const uint8_t *text, uint64_t n, uint32_t *sa, int sa_given,
+                       const b200sa_tree *h_out, uint64_t *num_nodes) {
+    if (!c) return B200SA_ERR_BAD_ARG;
+    if (n > B200SA_TREE_MAX_N) { c->last_error = "text longer than B200SA_TREE_MAX_N = 2^31-1 bytes"; return B200SA_ERR_TOO_LARGE; }
+    if (!h_out || !num_nodes || (n > 0 && (!text || !sa)) || !h_out->parent || !h_out->depth || !h_out->lo ||
+        !h_out->hi || !h_out->end || !h_out->nchildren)
+        return B200SA_ERR_BAD_ARG;
+    int rc = host_tree_inner(c, text, n, sa, sa_given, h_out, num_nodes);
+    if (rc != B200SA_OK) {
+        if (c->stream) cudaStreamSynchronize(c->stream);
+        cudaGetLastError();
+    }
+    return rc;
 }
 
 // ------------------------------------------------------------ multi-GPU: communicator + sharded LMS sort

@@ -614,6 +614,10 @@ struct AnsvLevels {
     uint64_t cnt[8];
     int nlev;
 };
+// STRICT: nearest value < v; otherwise nearest value <= v (block minima serve both).
+template <bool STRICT>
+__device__ __forceinline__ bool ansv_hit(uint32_t x, uint32_t v) { return STRICT ? x < v : x <= v; }
+template <bool STRICT>
 __device__ __forceinline__ uint32_t ansv_left(const AnsvLevels &L, uint64_t i, uint32_t v) {
     // climb: at level k, scan the siblings to the left inside the parent block; a block with min < v holds the answer
     uint64_t idx = i;
@@ -624,14 +628,14 @@ __device__ __forceinline__ uint32_t ansv_left(const AnsvLevels &L, uint64_t i, u
         bool found = false;
         while (j > first) {
             j--;
-            if (L.lv[k][j] < v) { found = true; break; }
+            if (ansv_hit<STRICT>(L.lv[k][j], v)) { found = true; break; }
         }
         if (found) {                       // descend: rightmost entry < v inside block j of level k
             while (k > 0) {
                 uint64_t base = j * 32, end = base + 32;
                 if (end > L.cnt[k - 1]) end = L.cnt[k - 1];
                 uint64_t q = end;
-                while (q > base) { q--; if (L.lv[k - 1][q] < v) break; }
+                while (q > base) { q--; if (ansv_hit<STRICT>(L.lv[k - 1][q], v)) break; }
                 j = q;
                 k--;
             }
@@ -646,6 +650,7 @@ __device__ __forceinline__ uint32_t ansv_left(const AnsvLevels &L, uint64_t i, u
         if (idx == 0) return ANSV_NONE;
     }
 }
+template <bool STRICT>
 __device__ __forceinline__ uint64_t ansv_right(const AnsvLevels &L, uint64_t i, uint32_t v, uint64_t n) {
     uint64_t idx = i;
     int k = 0;
@@ -654,13 +659,13 @@ __device__ __forceinline__ uint64_t ansv_right(const AnsvLevels &L, uint64_t i, 
         if (last > L.cnt[k]) last = L.cnt[k];
         uint64_t j = idx + 1;
         bool found = false;
-        for (; j < last; j++) if (L.lv[k][j] < v) { found = true; break; }
+        for (; j < last; j++) if (ansv_hit<STRICT>(L.lv[k][j], v)) { found = true; break; }
         if (found) {
             while (k > 0) {
                 uint64_t base = j * 32, end = base + 32;
                 if (end > L.cnt[k - 1]) end = L.cnt[k - 1];
                 uint64_t q = base;
-                while (q < end && !(L.lv[k - 1][q] < v)) q++;
+                while (q < end && !ansv_hit<STRICT>(L.lv[k - 1][q], v)) q++;
                 j = q;
                 k--;
             }
@@ -671,12 +676,14 @@ __device__ __forceinline__ uint64_t ansv_right(const AnsvLevels &L, uint64_t i, 
         if (k >= L.nlev) return n;
     }
 }
+// STRICT = false gives the previous / next smaller-or-equal values; a null nsv skips the right side.
+template <bool STRICT>
 __global__ void __launch_bounds__(BLK) k_ansv(AnsvLevels L, uint64_t n, uint32_t *psv, uint32_t *nsv) {
     uint64_t i = (uint64_t)blockIdx.x * BLK + threadIdx.x;
     if (i >= n) return;
     uint32_t v = L.lv[0][i];
-    psv[i] = ansv_left(L, i, v);
-    nsv[i] = (uint32_t)ansv_right(L, i, v, n);
+    psv[i] = ansv_left<STRICT>(L, i, v);
+    if (nsv) nsv[i] = (uint32_t)ansv_right<STRICT>(L, i, v, n);
 }
 
 }  // namespace b200sa
