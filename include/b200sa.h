@@ -62,7 +62,17 @@ int b200sa_build(b200sa_ctx *ctx, const uint8_t *text, uint64_t n, uint32_t *sa_
  * as called by SuffixTable::lcp_lens (src/table.rs:130-138):
  * lcp[0]=0, lcp[i]=|common byte prefix of suffix sa[i-1], suffix sa[i]|.
  * `sa` is checked to be a permutation of 0..n-1 (B200SA_ERR_BAD_ARG otherwise; the
- * reference would panic on an out-of-range index, src/table.rs:356-358). */
+ * reference would panic on an out-of-range index, src/table.rs:356-358).  Any permutation
+ * gives lcp_lens_quadratic's array; which path computes it:
+ *   - every pair first goes through a direct compare capped at 256 chars (when the text
+ *     packs to <= 16 symbols or is <= 32 MiB); if no pair reaches the cap, that is the result;
+ *   - otherwise the table is checked to be THE suffix array of the text (one inverse scatter
+ *     and one pass over the ranks, phase "lcp_sorted"); the suffix array takes the linear
+ *     Phi / PLCP path (Kasai), which is only valid on the sorted table;
+ *   - any other permutation (phase "lcp_unsorted") gets the reference's per-pair compare with
+ *     no cap: quadratic in the LCP values, like the reference, so slow on repetitive text.
+ * b200sa_lcp_dev and b200sa_lcp_sharded follow the same rules; the fused b200sa_build_lcp*
+ * built their table themselves and skip the check. */
 int b200sa_lcp(b200sa_ctx *ctx, const uint8_t *text, uint64_t n,
                const uint32_t *sa, uint32_t *lcp_out);
 
@@ -87,7 +97,9 @@ int b200sa_build_lcp_dev(b200sa_ctx *ctx, const uint8_t *d_text, uint64_t n,
  * Replaces SuffixTable::positions (src/table.rs:223-259) for a batch: query q
  * is bytes [q_off[q], q_off[q+1]) of d_queries; writes the SA range
  * [start[q], end[q]) whose entries are the match positions (SA order, as the
- * reference returns them). */
+ * reference returns them).  d_sa is trusted like SuffixTable::from_parts (not checked):
+ * on any permutation of 0..n-1 the result is what the reference's two binary searches
+ * return over that table. */
 int b200sa_positions_dev(b200sa_ctx *ctx, const uint8_t *d_text, uint64_t n,
                          const uint32_t *d_sa, const uint8_t *d_queries,
                          const uint64_t *d_q_off, uint32_t nq,
@@ -169,8 +181,11 @@ int b200sa_suffix_tree_dev(b200sa_ctx *ctx, const uint8_t *d_text, uint64_t n, c
 /* Host twin; the six arrays of h_out are host buffers of max(2n, 1) entries.
  *   sa_given == 0: SuffixTree::new -- SA and LCP are built on the device and the SA is written
  *                  to sa[0..n) (labels and terminals need it);
- *   sa_given != 0: SuffixTree::from_suffix_table -- sa[0..n) is read and checked to be a
- *                  permutation of 0..n-1 (B200SA_ERR_BAD_ARG otherwise), the LCP is computed
+ *   sa_given != 0: SuffixTree::from_suffix_table -- sa[0..n) is read and checked to be THE
+ *                  suffix array of the text: a permutation of 0..n-1 in suffix order
+ *                  (B200SA_ERR_BAD_ARG otherwise, with b200sa_last_error saying which; the
+ *                  tree kernels need the LCP intervals of the sorted table, and the
+ *                  reference's construction asserts on other tables), the LCP is computed
  *                  as b200sa_lcp does.
  * The LCP array stays on the device. */
 int b200sa_suffix_tree(b200sa_ctx *ctx, const uint8_t *text, uint64_t n, uint32_t *sa, int sa_given,
@@ -225,7 +240,11 @@ int b200sa_shard_lms_sort(b200sa_ctx *ctx, const uint8_t *d_shard, uint64_t len,
  * broadcast first; != 0: every rank already holds them.  Every rank computes Phi / PLCP for
  * its own range of text positions, the ranges are all-gathered, every rank turns its range of
  * ranks into LCP values, the slices are all-gathered: on return every rank holds the whole
- * lcp array, equal to lcp_lens_quadratic(text, table) (src/table.rs:348-361). */
+ * lcp array, equal to lcp_lens_quadratic(text, table) (src/table.rs:348-361).  Every rank
+ * checks that the table is a permutation and that it is the suffix array; all ranks hold the
+ * same table and reach the same verdict.  A permutation that is not the suffix array is not
+ * sharded: every rank computes the whole array with the uncapped per-pair compare (see
+ * b200sa_lcp) and no collective runs after the check. */
 int b200sa_lcp_sharded(b200sa_ctx *ctx, uint8_t *d_text, uint64_t n, uint32_t *d_sa, uint32_t *d_lcp,
                        int replicated, void *stream);
 

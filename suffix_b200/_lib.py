@@ -215,7 +215,8 @@ class Context:
 
     def suffix_tree(self, text: np.ndarray, sa: np.ndarray = None):
         """b200sa_suffix_tree -> (sa, {field: u32 array of the node count}).  sa=None builds the
-        table on the device (SuffixTree::new); a given table is checked (from_suffix_table)."""
+        table on the device (SuffixTree::new); a given table must be the suffix array of the
+        text (from_suffix_table), anything else raises B200SAError."""
         n = len(text)
         cap = max(2 * n, 1)
         out = {f: np.empty(cap, dtype=np.uint32) for f in TREE_FIELDS}

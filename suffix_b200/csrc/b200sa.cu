@@ -1002,8 +1002,42 @@ static int build_dev(b200sa_ctx *c, const uint8_t *d_text, uint64_t n, uint32_t 
     return B200SA_OK;
 }
 
+// k_lcp_direct on the packed text of the current call; pairs that reach `cap` (and could go on)
+// are counted in *capped.  cap >= n computes every pair in full.
+static void lcp_direct_launch(b200sa_ctx *c, uint32_t n32, const uint32_t *d_sa, uint32_t *d_lcp, uint32_t cap,
+                              uint32_t *capped) {
+    int lk = 2;       // runs of 32 ranks per warp = window gathers in flight per lane (2-bit text: 1 / 2 / 4 ->
+                      // 0.66 / 0.57 / 0.59 ms per 10^8 ranks; 4-bit text is best with 1)
+    if (const char *e = getenv("B200SA_LCP_K")) lk = atoi(e);
+    if (c->bits == 2 && lk == 4) LAUNCH(c, (k_lcp_direct<2, 4>), cdiv(n32, BLK * 4), c->ptext, n32, d_sa, d_lcp, cap, capped);
+    else if (c->bits == 2 && lk == 2) LAUNCH(c, (k_lcp_direct<2, 2>), cdiv(n32, BLK * 2), c->ptext, n32, d_sa, d_lcp, cap, capped);
+    else if (c->bits == 2) LAUNCH(c, (k_lcp_direct<2, 1>), cdiv(n32, BLK), c->ptext, n32, d_sa, d_lcp, cap, capped);
+    else if (c->bits == 4) LAUNCH(c, (k_lcp_direct<4, 1>), cdiv(n32, BLK), c->ptext, n32, d_sa, d_lcp, cap, capped);
+    else LAUNCH(c, (k_lcp_direct<8, 1>), cdiv(n32, BLK), c->ptext, n32, d_sa, d_lcp, cap, capped);
+}
+
+// Is a caller table that passed the permutation check THE suffix array of the n bytes at d_text?
+// inv (n u32) is scratch.  One scatter, one pass over the ranks, one word read back.
+static int sa_is_sorted(b200sa_ctx *c, const uint8_t *d_text, uint64_t n, const uint32_t *d_sa, uint32_t *inv,
+                        bool *sorted) {
+    uint32_t n32 = (uint32_t)n;
+    TRY(ensure(c, c->small, 4096));
+    uint32_t *bad = ptr<uint32_t>(c->small) + 14;
+    CU_TRY(c, cudaMemsetAsync(bad, 0, 4, c->stream));
+    LAUNCH(c, k_sa_inverse, cdiv(n, BLK), d_sa, n32, inv);
+    LAUNCH(c, k_sa_sorted, cdiv(n, BLK), d_text, n32, d_sa, inv, bad);
+    TRY(read_words(c, bad, 1));
+    *sorted = c->h_pin[0] == 0;
+    return B200SA_OK;
+}
+
+// reuse_pack: the table was built by this call (fused build_lcp*) and the packed text is ready.
+// Otherwise the table comes from the caller: it is checked to be a permutation, and before the
+// Phi / PLCP path (only valid on the sorted table) to be the suffix array; a permutation that is
+// not gets lcp_lens_quadratic's per-pair compare, uncapped.  require_sorted: reject a table that is
+// not the suffix array (B200SA_ERR_BAD_ARG) instead.
 static int lcp_dev(b200sa_ctx *c, const uint8_t *d_text, uint64_t n, const uint32_t *d_sa, uint32_t *d_lcp,
-                   bool reuse_pack) {
+                   bool reuse_pack, bool require_sorted = false) {
     if (n > B200SA_MAX_N) return B200SA_ERR_TOO_LARGE;
     if (n == 0) return B200SA_OK;
     uint32_t n32 = (uint32_t)n;
@@ -1050,25 +1084,41 @@ static int lcp_dev(b200sa_ctx *c, const uint8_t *d_text, uint64_t n, const uint3
         TRY(read_words(c, sm + 3, 1));
         TRY(pack_text(c, text, n, c->h_pin[0]));
     }
+    bool checked = false;
+    if (require_sorted) {
+        TRY(mark(c, "lcp_sorted"));
+        bool sorted = false;
+        TRY(sa_is_sorted(c, d_text, n, d_sa, ptr<uint32_t>(c->isa), &sorted));
+        if (!sorted) {
+            c->last_error = "table is not the suffix array of the text (adjacent suffixes out of order)";
+            return B200SA_ERR_BAD_ARG;
+        }
+        checked = true;
+    }
     // fast path: direct adjacent-pair compare when the text is L2-resident
     // (packed, or small); falls through to the linear path if any pair hits the cap
     if ((c->bits < 8 || n <= (32u << 20)) && !getenv("B200SA_LCP_LINEAR")) {
         TRY(mark(c, "lcp_direct"));
-        uint32_t *sm = ptr<uint32_t>(c->small);
         TRY(ensure(c, c->small, 4096));
-        sm = ptr<uint32_t>(c->small);
+        uint32_t *sm = ptr<uint32_t>(c->small);
         CU_TRY(c, cudaMemsetAsync(sm + 8, 0, 4, c->stream));
-        const uint32_t cap = 256;
-        int lk = 2;       // runs of 32 ranks per warp = window gathers in flight per lane (2-bit text: 1 / 2 / 4 ->
-                          // 0.66 / 0.57 / 0.59 ms per 10^8 ranks; 4-bit text is best with 1)
-        if (const char *e = getenv("B200SA_LCP_K")) lk = atoi(e);
-        if (c->bits == 2 && lk == 4) LAUNCH(c, (k_lcp_direct<2, 4>), cdiv(n, BLK * 4), c->ptext, n32, d_sa, d_lcp, cap, sm + 8);
-        else if (c->bits == 2 && lk == 2) LAUNCH(c, (k_lcp_direct<2, 2>), cdiv(n, BLK * 2), c->ptext, n32, d_sa, d_lcp, cap, sm + 8);
-        else if (c->bits == 2) LAUNCH(c, (k_lcp_direct<2, 1>), cdiv(n, BLK), c->ptext, n32, d_sa, d_lcp, cap, sm + 8);
-        else if (c->bits == 4) LAUNCH(c, (k_lcp_direct<4, 1>), cdiv(n, BLK), c->ptext, n32, d_sa, d_lcp, cap, sm + 8);
-        else LAUNCH(c, (k_lcp_direct<8, 1>), cdiv(n, BLK), c->ptext, n32, d_sa, d_lcp, cap, sm + 8);
+        lcp_direct_launch(c, n32, d_sa, d_lcp, 256u, sm + 8);
         TRY(read_words(c, sm + 8, 1));
         if (c->h_pin[0] == 0) {
+            TRY(mark(c, "end"));
+            CU_TRY(c, cudaGetLastError());
+            return B200SA_OK;
+        }
+    }
+    if (!reuse_pack && !checked) {
+        // a caller table about to take the linear path: Kasai's carry is only valid on the
+        // suffix array; any other permutation gets the reference's quadratic per-pair compare
+        TRY(mark(c, "lcp_sorted"));
+        bool sorted = false;
+        TRY(sa_is_sorted(c, d_text, n, d_sa, ptr<uint32_t>(c->isa), &sorted));
+        if (!sorted) {
+            TRY(mark(c, "lcp_unsorted"));
+            lcp_direct_launch(c, n32, d_sa, d_lcp, n32, ptr<uint32_t>(c->small) + 8);
             TRY(mark(c, "end"));
             CU_TRY(c, cudaGetLastError());
             return B200SA_OK;
@@ -1586,9 +1636,10 @@ static int host_tree_inner(b200sa_ctx *c, const uint8_t *text, uint64_t n, uint3
         TRY(mark(c, "h2d"));
         CU_TRY(c, cudaMemcpyAsync(c->text.p, text, n, cudaMemcpyHostToDevice, c->stream));
         if (sa_given) {
-            // SuffixTree::from_suffix_table: the table comes from the caller, lcp_dev checks it
+            // SuffixTree::from_suffix_table: the table comes from the caller, lcp_dev checks it; the
+            // tree kernels need the LCP intervals of the sorted table, so any other table is rejected
             CU_TRY(c, cudaMemcpyAsync(c->sa.p, sa, n * 4, cudaMemcpyHostToDevice, c->stream));
-            TRY(lcp_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa), ptr<uint32_t>(c->lcp), false));
+            TRY(lcp_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa), ptr<uint32_t>(c->lcp), false, true));
         } else {
             TRY(build_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa)));
             TRY(lcp_dev(c, ptr<uint8_t>(c->text), n, ptr<uint32_t>(c->sa), ptr<uint32_t>(c->lcp), n >= 2));
@@ -1962,6 +2013,23 @@ int b200sa_lcp_sharded(b200sa_ctx *c, uint8_t *d_text, uint64_t n, uint32_t *d_s
             return B200SA_ERR_BAD_ARG;
         }
         TRY(pack_text(c, d_text, n, c->h_pin[3]));
+    }
+    // ---- every rank: is the table the suffix array?  Phi / PLCP is only valid on the sorted table.
+    // Every rank holds the whole table, so all reach the same verdict; on a permutation that is not
+    // sorted each rank computes the whole array with the reference's per-pair compare, and no rank
+    // enters the collectives below.
+    TRY(mark(c, "lcp_sorted"));
+    {
+        bool sorted = false;
+        TRY(sa_is_sorted(c, d_text, n, d_sa, ptr<uint32_t>(c->isa), &sorted));
+        if (!sorted) {
+            TRY(mark(c, "lcp_unsorted"));
+            lcp_direct_launch(c, n32, d_sa, d_lcp, n32, sm + 8);
+            TRY(mark(c, "end"));
+            CU_TRY(c, cudaGetLastError());
+            CU_TRY(c, cudaStreamSynchronize(c->stream));
+            return end_call(c);
+        }
     }
     // ---- Phi and PLCP of this rank's text range
     TRY(mark(c, "lcps_plcp"));

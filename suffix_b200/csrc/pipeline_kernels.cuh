@@ -416,6 +416,30 @@ __global__ void __launch_bounds__(BLK) k_sa_validate_count(const uint32_t *__res
 __global__ void k_sa_validate_verdict(const uint32_t *cnt, uint32_t n, uint32_t *bad) {
     if (*cnt != n) atomicAdd(bad, 1u);
 }
+// Is a permutation (checked by k_sa_validate first) THE suffix array of the text?  The Phi / PLCP
+// path below is Kasai's algorithm: it relies on plcp[i] >= plcp[i-1] - 1, which only holds for the
+// sorted table.  Neighbour-order test with the inverse: for every adjacent pair (a, b) =
+// (sa[r-1], sa[r]), T[a] < T[b], or T[a] == T[b] and suffix a+1 precedes suffix b+1 (the empty
+// suffix precedes all).  *bad is set if any pair is out of order.
+__global__ void __launch_bounds__(BLK) k_sa_inverse(const uint32_t *__restrict__ sa, uint32_t n, uint32_t *inv) {
+    uint32_t r = blockIdx.x * BLK + threadIdx.x;
+    if (r < n) inv[sa[r]] = r;
+}
+__global__ void __launch_bounds__(BLK) k_sa_sorted(const uint8_t *__restrict__ text, uint32_t n,
+                                                   const uint32_t *__restrict__ sa, const uint32_t *__restrict__ inv,
+                                                   uint32_t *bad) {
+    uint32_t r = blockIdx.x * BLK + threadIdx.x;
+    bool wrong = false;
+    if (r > 0 && r < n) {
+        uint32_t a = sa[r - 1], b = sa[r];
+        uint32_t ca = __ldg(text + a), cb = __ldg(text + b);
+        if (ca != cb) wrong = ca > cb;
+        else if (a + 1 == n) wrong = false;          // "c" precedes "c..."
+        else if (b + 1 == n) wrong = true;
+        else wrong = inv[a + 1] >= inv[b + 1];
+    }
+    if (__ballot_sync(FULL, wrong) && lane_id() == 0) atomicOr(bad, 1u);
+}
 
 constexpr uint32_t PHI_NONE = 0xffffffffu;
 __global__ void __launch_bounds__(BLK) k_phi(const uint32_t *__restrict__ sa, uint32_t n, uint32_t *phi) {
@@ -498,7 +522,8 @@ __global__ void __launch_bounds__(BLK) k_plcp(const void *__restrict__ ptext, ui
     for (uint64_t i = i0 + 1; i < i1; i++) {
         uint32_t j = buf[i];
         if (j == PHI_NONE) { buf[i] = 0; h = 0; continue; }
-        uint32_t a = (uint32_t)i + h, b = j + h;     // a, b <= n (h never exceeds the shorter suffix)
+        uint32_t a = (uint32_t)i + h, b = j + h;     // a, b <= n: h never exceeds the shorter suffix on a
+                                                     // sorted table (k_sa_sorted checks caller tables)
         uint32_t limit = n - (a > b ? a : b);
         h += text_match<BITS>(ptext, a, b, limit);
         buf[i] = h;

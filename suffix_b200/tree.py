@@ -37,7 +37,8 @@ class SuffixTree:
 
     @classmethod
     def from_suffix_table(cls, st: SuffixTable) -> "SuffixTree":
-        """SuffixTree::from_suffix_table: the table is checked to be a permutation."""
+        """SuffixTree::from_suffix_table: the table is checked to be the suffix array of the
+        text; any other table raises B200SAError (B200SA_ERR_BAD_ARG)."""
         return cls(st.text(), st._device, _table=np.asarray(st.table()))
 
     def text(self) -> bytes:
